@@ -24,6 +24,10 @@ the max-over-ranks time).
 
 `--impl reference` times the CPU stand-in of the reference path (libcrypto when built, else the oracle's C port; the Go
 reference itself cannot be built here: no Go toolchain, un-vendored x/crypto) on all host threads.
+
+`--dump-outputs DIR` writes what the `value` leg (or, with `--impl reference`, the CPU stand-in) returned in its last timed
+step as DIR/status.npy: the per-signature status bytes as float32 (DIR/status_rank<r>.npy per rank when N > 1).  The
+inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -117,6 +121,14 @@ class ClockSampler:
                 "reasons": reasons, "samples": len(sm)}
 
 
+def dump_outputs(out_dir, arrays, rank, world):
+    """Writes each array as out_dir/<name>.npy in float32 (exact for the byte-sized statuses dumped here)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ("_rank%d" % rank if world > 1 else "") + ".npy"), np.asarray(a, np.float32))
+
+
 def w_pool_clean(w):
     """The genuinely signed, known-key subset of a config-2 batch, as a pool for config 3."""
     import numpy as np
@@ -159,6 +171,8 @@ def run_reference(args, rank, world):
         rate, st = cpu_verify(w, threads, 1, kind)
     dt = time.perf_counter() - t0
     assert (st == w["expect"]).all()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"status": st}, rank, world)
     v = ITEMS * args.steps / dt
     port_rate, _ = cpu_verify(w, threads, 1, "port")
     print(json.dumps({
@@ -258,6 +272,8 @@ def run_gpu(args, rank, local_rank, world):
     gpu_launches = eng.stats()["launches"] - launches0
     for c in range(min(copies, args.steps)):
         assert np.array_equal(d_st[c].cpu().numpy(), w["expect"]), "device-resident results differ from expectation"
+    if args.dump_outputs:                    # the buffer the last timed step wrote, before the sustained leg reuses it
+        dump_outputs(args.dump_outputs, {"status": d_st[(args.steps - 1) % copies].cpu().numpy()}, rank, world)
     # the same leg for >= SUSTAIN seconds: what the clocks do under a seconds-long integer load
     n_sus = max(args.steps, int(args.sustain * 1e3 / max(dev_ms / args.steps, 1e-3)) + 1)
     barrier()
@@ -437,10 +453,9 @@ def run_gpu(args, rank, local_rank, world):
     def cstep():
         L_.check(eng._lib.bftq_collective_verify_batch(krc._h, C.cast(carr, C.c_void_p), 1, vp(cmem), 16, vp(cpin[0]), vp(cpin[1]), vp(cpin[2]), vp(cpin[3]), NC, vp(cerr)))
     cstep()
-    csteps = max(3, min(args.steps, 5))
     barrier()
     t0 = time.perf_counter()
-    for _ in range(csteps):
+    for _ in range(args.steps):
         cstep()
     coll_s = time.perf_counter() - t0
     barrier()
@@ -468,13 +483,12 @@ def run_gpu(args, rank, local_rank, world):
     def qstep():
         eng.verify_tally_batch_dev(quorum, dq["off"], dq["idx"], dq["sig"], dq["dig"], M, NQ, dq_st, dq_bits, d_pre=dq["pre"],
                                    d_ts=dq["ts"], d_value_id=dq["val"], d_winner=dq_win, stream=stream.cuda_stream)
-    qsteps = max(3, min(args.steps, 5))
     for _ in range(2):
         qstep()
     barrier()
     q0, q1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     q0.record(stream)
-    for _ in range(qsteps):
+    for _ in range(args.steps):
         qstep()
     q1.record(stream)
     stream.synchronize()
@@ -522,10 +536,9 @@ def run_gpu(args, rank, local_rank, world):
         eng5.verify_read_batch(quorum5, pin5["op_off"], pin5["key_idx"], pin5["sig"], pin5["digest"], pin5["ts"], pin5["value_id"],
                                pre_status=pin5["pre_status"], out_status=out5[0], out_decision=out5[1], out_winner=out5[2], out_decided_at=out5[3])
     q5step()
-    q5steps = max(2, min(args.steps, 3))
     barrier()
     t0 = time.perf_counter()
-    for _ in range(q5steps):
+    for _ in range(args.steps):
         q5step()
     torch.cuda.synchronize(dev)
     q5_s = time.perf_counter() - t0
@@ -564,11 +577,10 @@ def run_gpu(args, rank, local_rank, world):
         return read_responses_batch(kr6, qcs6, ra["op_off"], ra["peer_ids"], None, ra["nonces"], pre_status=ra["pre_status"], blobs=pin6)
     q6step()
     s60 = eng6.stats()
-    q6steps = max(2, min(args.steps, 3))
     barrier()
     t0 = time.perf_counter()
     q6_each = []
-    for _ in range(q6steps):
+    for _ in range(args.steps):
         t1 = time.perf_counter()
         got6 = q6step()
         q6_each.append((time.perf_counter() - t1) * 1e3)
@@ -582,8 +594,8 @@ def run_gpu(args, rank, local_rank, world):
                                                  ra["ts"], ra["value_id"])
         assert np.array_equal(got6["decision"], rd) and np.array_equal(got6["winner"], rw) and np.array_equal(got6["decided_at"], ra_), \
             "raw-answer decisions differ from the oracle"
-    q6_info = {"bytes_per_answer": int(off6[-1]) // max(1, int((ra["pre_status"] == 0).sum())), "h2d_bytes_per_step": (s61["h2d_bytes"] - s60["h2d_bytes"]) // q6steps,
-               "gpu_parsed": (s61["msg_gpu_items"] - s60["msg_gpu_items"]) // q6steps, "host_parsed": (s61["msg_host_items"] - s60["msg_host_items"]) // q6steps,
+    q6_info = {"bytes_per_answer": int(off6[-1]) // max(1, int((ra["pre_status"] == 0).sum())), "h2d_bytes_per_step": (s61["h2d_bytes"] - s60["h2d_bytes"]) // args.steps,
+               "gpu_parsed": (s61["msg_gpu_items"] - s60["msg_gpu_items"]) // args.steps, "host_parsed": (s61["msg_host_items"] - s60["msg_host_items"]) // args.steps,
                "decisions": {k: int((got6["decision"] == v).sum()) for k, v in (("value", 0), ("rejected", 1), ("exhausted", 2))}}
     kr6.close()
     for a in pin6:
@@ -626,11 +638,11 @@ def run_gpu(args, rank, local_rank, world):
         stream.synchronize()
         a0, a1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         a0.record(stream)
-        for _ in range(3):
+        for _ in range(args.steps):
             estep()
         a1.record(stream)
         stream.synchronize()
-        e_ms = a0.elapsed_time(a1) / 3
+        e_ms = a0.elapsed_time(a1) / args.steps
         bad = int((de_st != 0).sum())
         assert bad == len(range(0, NE, 97)), "Ed25519 statuses differ from expectation"
         # Lagrange combine, 2t = 10 of n = 15 shares over the P-256 group order: host API incl. copies, and K3 alone
@@ -727,21 +739,21 @@ def run_gpu(args, rank, local_rank, world):
                      "api": "bftq_rsa_verify_batch (flat tuples: key index, padded signature, precomputed digest; pinned host buffers), "
                             "%d concurrent callers" % NCALLERS,
                      "ms_per_step": e2e_ms / args.steps},
-        "collective": {"metric": "collective_signature_verifies_per_sec", "value": NC * world * csteps / (coll_ms * 1e-3), "unit": "collective verifies/s",
-                       "signature_verifies_per_sec": NC * NSIG * world * csteps / (coll_ms * 1e-3), "steps": csteps, "ms_per_step": coll_ms / csteps,
+        "collective": {"metric": "collective_signature_verifies_per_sec", "value": NC * world * args.steps / (coll_ms * 1e-3), "unit": "collective verifies/s",
+                       "signature_verifies_per_sec": NC * NSIG * world * args.steps / (coll_ms * 1e-3), "steps": args.steps, "ms_per_step": coll_ms / args.steps,
                        "api": "bftq_collective_verify_batch = crypto.CollectiveSignature.Verify's batch form (crypto_pgp.go:485-500): TBSS strings + concatenated "
                               "OpenPGP signature packets in page-locked host blobs in, nil / ErrInsufficientNumberOfSignatures out; packets framed on the host, "
                               "K0 + K1 + K2 (IsSufficient) on the GPU",
                        "config": {"workload": "%d collective signatures x 11 packets by members of a 16-node clique (f = 5, suff = 11), 2%% of the packets corrupted" % NC,
                                   "accepted_rank0": coll_accept, "data": "synthetic; packets drawn from 8 x 16 genuine signatures"}},
-        "quorum_ops": {"metric": "quorum_certified_read_ops_per_sec", "value": M * world * qsteps / (q_ms * 1e-3), "unit": "ops/s",
-                       "verifies_per_sec": NQ * world * qsteps / (q_ms * 1e-3), "steps": qsteps, "ms_per_step": q_ms / qsteps,
+        "quorum_ops": {"metric": "quorum_certified_read_ops_per_sec", "value": M * world * args.steps / (q_ms * 1e-3), "unit": "ops/s",
+                       "verifies_per_sec": NQ * world * args.steps / (q_ms * 1e-3), "steps": args.steps, "ms_per_step": q_ms / args.steps,
                        "config": {"workload": "batch 65536 read ops x 16-replica quorum, verify + wotqs read tally (BASELINE configs[2]), device-resident",
                                   "quorum": "n=16 f=5 READ threshold 6", "accepted_ops_rank0": accepted,
                                   "data": "synthetic; 1,048,576 tuples drawn from a pool of 65,536 genuine signatures"},
                        "kernels_per_step": 2,
-                       "e2e": {"metric": "quorum_certified_read_ops_per_sec", "value": M5 * world * q5steps / (q5_ms * 1e-3), "unit": "ops/s",
-                               "verifies_per_sec": NQ5 * world * q5steps / (q5_ms * 1e-3), "steps": q5steps, "ms_per_step": q5_ms / q5steps,
+                       "e2e": {"metric": "quorum_certified_read_ops_per_sec", "value": M5 * world * args.steps / (q5_ms * 1e-3), "unit": "ops/s",
+                               "verifies_per_sec": NQ5 * world * args.steps / (q5_ms * 1e-3), "steps": args.steps, "ms_per_step": q5_ms / args.steps,
                                "h2d_bytes_per_step": h2d5, "d2h_bytes_per_step": d2h5,
                                "api": "bftq_verify_read_batch: flat tuples in page-locked host memory in, per-tuple status + per-op Client.Read decision "
                                       "(value / rejected / exhausted, winner, decided_at) out; chunked H2D + K1 + K2 + D2H inside the timed region",
@@ -753,10 +765,10 @@ def run_gpu(args, rank, local_rank, world):
                                                        "(workload.HARD_MIX); responses arrive in seeded random order",
                                           "decisions_rank0": dec_hist, "checked": "statuses vs expectation on every rank; decisions vs the C oracle on rank 0",
                                           "data": "synthetic; tuples drawn from a pool of %d genuine signatures over 31 keys" % args.pool5}},
-                       "e2e_packets": {"metric": "quorum_certified_read_ops_per_sec", "value": M6 * world * q6steps / (q6_ms * 1e-3), "unit": "ops/s",
-                                       "answers_per_sec": N6 * world * q6steps / (q6_ms * 1e-3), "steps": q6steps, "ms_per_step": q6_ms / q6steps, "ms_each_step_rank0": [round(x, 3) for x in q6_each],
+                       "e2e_packets": {"metric": "quorum_certified_read_ops_per_sec", "value": M6 * world * args.steps / (q6_ms * 1e-3), "unit": "ops/s",
+                                       "answers_per_sec": N6 * world * args.steps / (q6_ms * 1e-3), "steps": args.steps, "ms_per_step": q6_ms / args.steps, "ms_each_step_rank0": [round(x, 3) for x in q6_each],
                                        "h2d_bytes_per_step": int(q6_info["h2d_bytes_per_step"]), "bytes_per_answer": q6_info["bytes_per_answer"],
-                                       "h2d_gbps_achieved": q6_info["h2d_bytes_per_step"] * q6steps / (q6_ms * 1e-3) / 1e9,
+                                       "h2d_gbps_achieved": q6_info["h2d_bytes_per_step"] * args.steps / (q6_ms * 1e-3) / 1e9,
                                        "api": "bftq_read_responses_batch: the decrypted transport answers (one-pass signature, partial-length literal data, signature) in "
                                               "page-locked host memory in, per-answer status + per-op Client.Read decision out; message parsing, de-chunking, nonce check, "
                                               "packet.Parse, SHA-256, RSA verify and the tally all on the GPU",
@@ -837,6 +849,7 @@ def main():
     ap.add_argument("--ops6", type=int, default=8192, help="read operations per GPU in the raw-answer leg")
     ap.add_argument("--coll-items", type=int, default=16384, help="collective signatures per step in the server-side leg")
     ap.add_argument("--skip-ed25519", action="store_true", help="skip the BASELINE configs[3] secondary measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's status bytes to DIR/status.npy (float32)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
