@@ -232,11 +232,16 @@ _HASHLIB = {1: "md5", 2: "sha1", 3: "ripemd160", 8: "sha256", 9: "sha384", 10: "
 
 
 def raw_rsa_sign(k, hash_id: int, digest: bytes) -> int:
-    """EMSA-PKCS1-v1_5 signature by textbook exponentiation (k carries d): works for digests OpenSSL refuses to sign."""
+    """EMSA-PKCS1-v1_5 signature by textbook exponentiation (k carries d): works for digests OpenSSL refuses to sign.
+    With the primes in k the exponentiation goes through the CRT (same signature, about four times faster)."""
     t = bytes.fromhex(_DIGESTINFO[hash_id]) + digest
     klen = (k["n"].bit_length() + 7) // 8
-    em = b"\x00\x01" + b"\xff" * (klen - len(t) - 3) + b"\x00" + t
-    return pow(int.from_bytes(em, "big"), k["d"], k["n"])
+    em = int.from_bytes(b"\x00\x01" + b"\xff" * (klen - len(t) - 3) + b"\x00" + t, "big")
+    if "p" not in k:
+        return pow(em, k["d"], k["n"])
+    p, q = k["p"], k["q"]
+    sp, sq = pow(em, k["d"] % (p - 1), p), pow(em, k["d"] % (q - 1), q)
+    return sq + q * ((sp - sq) * pow(q, -1, p) % p)
 
 
 def canonical_text(data: bytes) -> bytes:
